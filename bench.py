@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the TokenPacker projector hot path on B200 (contract: see the task brief / DESIGN.md §Measurement).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload projector|hd5|train]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload projector|hd5|train] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 One "step" = one TokenPacker.forward over one batch of synthetic CLIP features per GPU.  Workload at every N:
@@ -202,8 +202,8 @@ def cpu_reference_run(steps: int, warmup: int, crops: int):
             torch_port.forward(params, x0[:1], xm[:1], SCALE)
         single_ms = (time.perf_counter() - t0) / 5 * 1e3
     return {"value": crops * TOKENS_PER_CROP / dt, "unit": UNIT, "cores": int(torch.get_num_threads()), "kind": "port",
-            "pinned": "oracle/torch_port.py is held to fixtures generated by the reference module itself (tests/golden, < 1e-6) and to live "
-                      "runs of the reference where /root/reference is mounted (tests/test_reference_live.py)",
+            "pinned": "oracle/torch_port.py is held to fixtures generated by the reference module itself (tests/golden, < 1e-6) and to the "
+                      "reference's answers on seeded random cases (tests/test_reference_live.py)",
             "configs0_single_image_ms": single_ms,
             "sample": f"{crops} crops/step x {steps} steps of the configs[1] workload (fp32, torch {torch.__version__} CPU ops, "
                       f"oracle/torch_port.py restatement of builder.py:107-137; best of pool sizes {cands} on {avail} visible cores), {dt * 1e3:.1f} ms/step"}, dt
@@ -363,7 +363,7 @@ def run_hd5(args, rank, world, dev, dist):
 # ----------------------------------------------------------------------------------------------------------------------
 # training step (SURVEY.md §8f N1)
 # ----------------------------------------------------------------------------------------------------------------------
-def train_measure(model, x0, xm, steps=10):
+def train_measure(model, x0, xm, steps=10, warmup=3):
     """Forward + backward of the projector at the configs[1] batch (the reference trains this module through autograd,
     train.py:950-958) next to PyTorch eager autograd over the reference's op sequence (oracle/torch_port.py, bf16, same GPU)."""
     from tokenpacker_b200._lib import lib
@@ -381,7 +381,7 @@ def train_measure(model, x0, xm, steps=10):
         return out
 
     go = torch.randn(x0.shape[0], model.num_queries, model.hidden_size, device=x0.device).to(torch.bfloat16) * 0.01
-    for _ in range(3):
+    for _ in range(warmup):
         step()
     torch.cuda.synchronize()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -469,6 +469,19 @@ def hd_tile_measure(dev, peaks):
             "achieved_gbs": bytes_alg / (ms * 1e-3) / 1e9, "peak_gbs": peaks["hbm_gbs"], "frac": bytes_alg / (ms * 1e-3) / 1e9 / peaks["hbm_gbs"]}
 
 
+DUMP_ROWS = 2048                 # of the N_CROPS x TOKENS_PER_CROP = 9,216 output rows: 2048 x 4096 fp32 = 32 MiB
+
+
+def dump_outputs(out, path):
+    """What the timed forward returned in its last step, for comparing two builds output for output: a fixed seeded sample
+    of DUMP_ROWS whole token rows (ascending row order, fp32) and the fp64 sum of every row of the full output."""
+    os.makedirs(path, exist_ok=True)
+    rows = out.reshape(-1, out.shape[-1])
+    pick = torch.randperm(rows.shape[0], generator=torch.Generator().manual_seed(0))[:DUMP_ROWS].sort().values
+    np.save(os.path.join(path, "out_sampled_rows.npy"), rows[pick.to(rows.device)].float().cpu().numpy())
+    np.save(os.path.join(path, "out_row_sums.npy"), out.double().sum(dim=-1).cpu().numpy())
+
+
 def bind_numa(local_rank):
     try:
         from tokenpacker_b200.numa import bind_to_gpu_node
@@ -490,7 +503,14 @@ def main():
     ap.add_argument("--no-e2e", action="store_true", help="skip the host-buffer end-to-end leg (profiling runs)")
     ap.add_argument("--no-extras", action="store_true", help="skip the sustained / hd5 / train / eager records (profiling runs)")
     ap.add_argument("--sustained-seconds", type=float, default=2.0)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="projector workload: after the timed steps, write rank 0's output of the last timed step to DIR/*.npy "
+                         "(a seeded sample of whole rows, plus every row's sum)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "projector"):
+        ap.error("--dump-outputs applies to --impl ours --workload projector")
     args.warmup = max(args.warmup, 3)
 
     if args.impl == "reference":
@@ -537,10 +557,10 @@ def main():
     xm = torch.randn(N_CROPS, 576, 4096, device=dev, generator=g).to(torch.bfloat16)
 
     if args.workload == "train":
-        rec = train_measure(model, x0, xm, steps=max(3, min(args.steps, 50)))
+        rec = train_measure(model, x0, xm, steps=args.steps, warmup=args.warmup)
         if rank == 0:
             print(json.dumps({"metric": "projector_train_step_ms", "value": rec["fwd_bwd_ms"], "unit": "ms", "n_gpus": world, "steps": rec["steps"],
-                              "warmup": 3, "ms_per_step": rec["fwd_bwd_ms"], "higher_is_better": False, "scaling": "weak", "dtype": "bf16",
+                              "warmup": args.warmup, "ms_per_step": rec["fwd_bwd_ms"], "higher_is_better": False, "scaling": "weak", "dtype": "bf16",
                               "data": "synthetic", "config": {"workload": "configs[1] batch, forward + backward"}, "train": rec}), flush=True)
         if dist is not None:
             dist.destroy_process_group()
@@ -587,6 +607,8 @@ def main():
         ms_per_step, clocks, launches, out = timed_steps(args.steps, True)
     value = tokens_per_step / (ms_per_step * 1e-3)
     assert torch.isfinite(out.float()).all()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(out, args.dump_outputs)
     region_s = ms_per_step * args.steps * 1e-3
     regime = "sustained" if region_s >= 1.0 else "burst"
 
